@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- aligned bases / second through pileup + consensus (BASELINE.json's metric).
 
-    python bench.py --gpus 1 --steps 20 --warmup 5             # this engine, 1 GPU
+    python bench.py --gpus 1 --warmup 5                        # this engine, 1 GPU, >= 0.5 s of timed steps
     torchrun ... bench.py --gpus N ...                         # sharded over N GPUs (one process per GPU)
     python bench.py --impl reference ...                       # the reference's own CPU functions, same metric
 
@@ -18,9 +18,10 @@ slot is shared, nothing is reduced).  Other workloads: --workload (cfg2, cfg3, c
 
 Numbers on the JSON line:
   value         whole-job aligned bases/s with the flattened reads already resident in HBM; CUDA events on the
-                launch stream, max over ranks, over >= 0.5 s of back-to-back steps (`steps_timed`; `steps` echoes
-                the request); `step_ms` = min / median / p90 / max of the individual steps.
-  e2e           the same metric from HOST buffers: N = 1 through the C-ABI call kdl_ctx_consensus (pinned host
+                launch stream, max over ranks, over exactly --steps back-to-back steps or, without --steps, as
+                many as cover >= 0.5 s of device time (`steps_timed`; `steps` echoes the request);
+                `step_ms` = min / median / p90 / max of the individual steps.
+  e2e           the same metric from HOST buffers, mean over max(3, min(steps_timed, 10)) calls: N = 1 through the C-ABI call kdl_ctx_consensus (pinned host
                 buffers in, H2D + kernels + D2H of the call bytes inside the timed region); N > 1 through the whole
                 sharded job (every rank's H2D of its shard + K1 + exchange + vote + D2H of the complete call bytes).
   roofline      dominant kernel (K0 + K1) against the measured HBM copy bandwidth (MEASURED_PEAKS.json).
@@ -28,6 +29,12 @@ Numbers on the JSON line:
   cpu_baseline  the reference's own functions on this box's host CPU, bounded sample (see --impl reference).
 Inputs are larger than L2 (126 MB) for the cfg4 / cfg5 workloads (no flush needed); the small ones (cfg2, cfg3)
 fit in L2 and say so in config.l2_policy.
+
+--dump-outputs DIR writes what the last timed step computed -- the count table, the insertion-event rows and the
+call bytes a caller of pileup + vote receives (N > 1: the call bytes) -- as DIR/<name>.npy in float32 (float64
+where float32 would round), at most DUMP_BYTES in all: an array that does not fit keeps a fixed, seeded sample of
+its slots / rows, and DIR/<name>_index.npy says which.  The workloads are generated from fixed seeds, so two builds
+run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -50,7 +57,8 @@ if ROOT not in sys.path:
 
 METRIC = "aligned bases/sec through pileup+consensus"
 UNIT = "aligned_bases/s"
-MIN_TIMED_S = 0.5  # the headline rests on at least this much device time
+MIN_TIMED_S = 0.5  # without --steps, the headline rests on at least this much device time
+DUMP_BYTES = 60_000_000  # --dump-outputs: the data of all arrays together (each .npy adds a 128-byte header)
 
 WORKLOADS = {
     # name: (contig lengths, depth, fraction of indel/clip reads or "cfg3", N > 1 partition)
@@ -266,7 +274,7 @@ def cpu_reference_pass(ref, recs, window):
 
 
 def cpu_reference_sample(batch, target_bases=5.0e7):
-    """The reference's OWN functions (unmodified kindel/kindel.py, staged under baseline/_ref by
+    """The reference's OWN functions (unmodified kindel/kindel.py, staged under oracle/_ref by
     oracle/stage_reference.py; loaded through oracle/refload.py's import stubs): parse_records +
     consensus_sequence (kindel.py:21-128, 384-430) on a bounded sample, single core -- the reference has no
     parallelism (kindel/kindel.py:1-14 imports no threading / multiprocessing).  Falls back to the
@@ -367,24 +375,29 @@ def run_reference(args):
 
 
 # ----------------------------------------------------------------------------------- GPU arm
-def time_steps(step, steps_req, warmup, torch, dist, world, dev, min_seconds=MIN_TIMED_S):
-    """W warm-up steps, then R >= steps_req back-to-back steps covering >= min_seconds of device time; one CUDA
-    event triple per step (dispersion, K1 / K2 split) -- the region is bracketed by the first and last events."""
+def time_steps(step, steps, warmup, torch, dist, world, dev, min_seconds=MIN_TIMED_S):
+    """W warm-up steps, then exactly `steps` back-to-back steps -- or, if `steps` is None, as many as cover
+    >= min_seconds of device time at the step time of 3 more untimed steps; one CUDA event triple per step
+    (dispersion, K1 / K2 split) -- the region is bracketed by the first and last events."""
     for _ in range(warmup):
         step()
     torch.cuda.synchronize()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for _ in range(3):  # estimate the step time to size the timed region
-        step()
-    e1.record()
-    torch.cuda.synchronize()
-    est_ms = max(e0.elapsed_time(e1) / 3, 1e-3)
-    reps = min(max(steps_req, int(math.ceil(min_seconds * 1e3 / est_ms))), 20000)
-    if world > 1:  # every rank must run the same number of steps
-        t = torch.tensor([reps], dtype=torch.int64, device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        reps = int(t.item())
+    if steps is not None:
+        reps = max(1, steps)
+    else:
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(3):
+            step()
+        e1.record()
+        torch.cuda.synchronize()
+        est_ms = max(e0.elapsed_time(e1) / 3, 1e-3)
+        reps = min(int(math.ceil(min_seconds * 1e3 / est_ms)), 20000)
+        if world > 1:  # every rank must run the same number of steps
+            t = torch.tensor([reps], dtype=torch.int64, device=dev)
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)
+            reps = int(t.item())
+    if world > 1:
         dist.barrier()
     ev = [tuple(torch.cuda.Event(enable_timing=True) for _ in range(3)) for _ in range(reps)]
     ev_end = torch.cuda.Event(enable_timing=True)
@@ -402,6 +415,29 @@ def time_steps(step, steps_req, warmup, torch, dist, world, dev, min_seconds=MIN
     k2_ms = [e[1].elapsed_time(e[2]) for e in ev]
     return {"reps": reps, "total_ms": total_ms, "step_ms": step_ms, "k1_ms": statistics.mean(k1_ms),
             "k2_ms": statistics.mean(k2_ms), "out": out}
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """arrays: {name: (numpy array, axis along which it may be sampled)} -> out_dir/<name>.npy.  Smaller arrays are
+    written whole; the budget left is shared among the larger ones, which keep a seeded sample along their axis."""
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1][0].size)
+    left = budget
+    for i, (name, (a, axis)) in enumerate(items):
+        a = np.asarray(a)
+        dt = np.float32 if a.size == 0 or np.abs(a).max() < 2 ** 24 else np.float64
+        share = left // (len(items) - i)
+        n = a.shape[axis]
+        per = np.dtype(dt).itemsize * (a.size // max(n, 1))
+        if per * n > share:
+            k = max(1, share // (per + 8))  # + the float64 index of each kept slot / row
+            idx = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+            a = np.take(a, idx, axis=axis)
+            np.save(os.path.join(out_dir, name + "_index.npy"), idx.astype(np.float64))
+            left -= 8 * k
+        out = np.ascontiguousarray(a, dtype=dt)
+        np.save(os.path.join(out_dir, name + ".npy"), out)
+        left -= out.nbytes
 
 
 def oracle_digest(batch, torch, dist, world, dev, min_depth=1):
@@ -454,23 +490,23 @@ def run_native(args):
                 # a fresh pileup into a reused table: nothing is memset, K1 overwrites the weight columns
                 if timers:
                     timers[0].record()
-                engine.pileup(db, check=False, table=table)
+                counts, events = engine.pileup(db, check=False, table=table)
                 if timers:
                     timers[1].record()
-                out = engine.vote(table.t, 1, out=calls_buf)
+                calls = engine.vote(table.t, 1, out=calls_buf)
                 if timers:
                     timers[2].record()
-                return out
+                return {"counts": counts, "events": events, "calls": calls}
             return batch, total, sharding, step, None
         from kindel_b200 import distributed
 
         sc = distributed.ShardedConsensus(batch, dev, mode=args.exchange)
 
         def step(timers=None):
-            out = sc.step(1, timers)
+            calls = sc.step(1, timers)
             if timers:
                 timers[2].record()
-            return out
+            return {"calls": calls}
         return batch, total, sharding, step, sc
 
     batch, total_bases, sharding, step, sc = build_case(args.scaling)
@@ -484,9 +520,12 @@ def run_native(args):
     tm = time_steps(step, args.steps, args.warmup, torch, dist, world, dev)
     launches = lib.kdl_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
-    launches_per_step = launches / (args.warmup + 3 + tm["reps"])
+    launches_per_step = launches / (args.warmup + (0 if args.steps is not None else 3) + tm["reps"])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {name: (t.cpu().numpy(), 1 if name == "counts" else 0)
+                                         for name, t in tm["out"].items()})
     # parity of what the timed loop produced (outside the timed region)
-    got = hashlib.sha256(tm["out"].cpu().numpy().tobytes()).hexdigest()
+    got = hashlib.sha256(tm["out"]["calls"].cpu().numpy().tobytes()).hexdigest()
     want = oracle_digest(batch, torch, dist, world, dev)
     t = torch.tensor([tm["total_ms"], tm["k1_ms"], tm["k2_ms"], 0.0 if got == want else 1.0], dtype=torch.float64,
                      device=dev)
@@ -498,7 +537,7 @@ def run_native(args):
     step_q = quantiles(tm["step_ms"])
 
     # ---- e2e from pinned HOST buffers ---------------------------------------------------------------
-    n_e2e = max(3, min(args.steps, 10))
+    n_e2e = max(3, min(tm["reps"], 10))
     if world == 1:
         ctx = engine.HostContext(local)
         pinned = {}
@@ -562,7 +601,7 @@ def run_native(args):
     if world > 1 and args.scaling == "weak" and not args.no_strong:
         sb, s_total, s_sharding, s_step, s_sc = build_case("strong")
         stm = time_steps(s_step, args.steps, args.warmup, torch, dist, world, dev, min_seconds=0.25)
-        s_got = hashlib.sha256(stm["out"].cpu().numpy().tobytes()).hexdigest()
+        s_got = hashlib.sha256(stm["out"]["calls"].cpu().numpy().tobytes()).hexdigest()
         s_par = s_got == oracle_digest(sb, torch, dist, world, dev)
         tt = torch.tensor([stm["total_ms"], stm["k1_ms"], 0.0 if s_par else 1.0], dtype=torch.float64, device=dev)
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -606,7 +645,7 @@ def run_native(args):
                          "algorithmic_bytes_per_launch": k1_bytes, "kernel_ms": k1_ms_max},
             "kernels_ms": {"k0_k1_pileup": k1_ms_max, "k2_vote_or_exchange": k2_ms_max,
                            "k2_vote_gbs": (k2_bytes / (k2_ms_max * 1e-3) / 1e9) if world == 1 and k2_ms_max else None},
-            "e2e": e2e, "gpu_launches": int(round(launches_per_step * args.steps)),
+            "e2e": e2e, "gpu_launches": int(round(launches_per_step * tm["reps"])),
             "gpu_launches_per_step": launches_per_step, "clocks": clocks,
         }
         if strong is not None:
@@ -626,11 +665,15 @@ def run_native(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps, exactly (default: as many as cover >= 0.5 s of device time; --impl reference: 20)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", choices=["native", "reference"], default="native")
     ap.add_argument("--workload", choices=sorted(WORKLOADS), default="cfg4_5Mb_200x")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32/float64, seeded sample "
+                         "of arrays beyond the size budget)")
     ap.add_argument("--no-strong", action="store_true", help="N > 1: skip the strong-scaling measurement beside the weak one")
     ap.add_argument("--scaling", choices=["weak", "strong"], default="weak",
                     help="N > 1: weak = the full per-GPU workload on every rank (N x deeper in total); "
@@ -643,6 +686,8 @@ def main():
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
+        if args.steps is None:
+            args.steps = 20
         return run_reference(args)
     return run_native(args)
 

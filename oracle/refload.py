@@ -1,17 +1,17 @@
 """TEST INFRASTRUCTURE ONLY -- loads the UNMODIFIED reference (bede/kindel) for pinning the oracle.
 
-This module exists only in service of `oracle/make_golden.py` and the `-m "not gpu"` tests that run
-in the build container: it imports `/root/reference/kindel/kindel.py` exactly as it lies on disk
-(never copied into this repo) by stubbing the three third-party imports that are not installed
-here (`simplesam`, `dnaio`, `argh`; reference `kindel/kindel.py:3,9,14`, `kindel/cli.py:2`) and
+This module exists only in service of the golden-data generators (`oracle/make_*golden.py`) and of
+`bench.py`'s CPU legs: it imports `kindel/kindel.py` of a reference checkout (KINDEL_REFERENCE_ROOT)
+exactly as it lies on disk (never copied into this repo) by stubbing the three third-party imports that
+need not be installed (`simplesam`, `dnaio`, `argh`; reference `kindel/kindel.py:3,9,14`, `kindel/cli.py:2`) and
 by feeding it records from a small stdlib (gzip + struct) BAM/SAM decoder that produces the four
 attributes the pileup consumes (`.pos`, `.mapped`, `.seq`, `.cigars`; reference
 `kindel/kindel.py:42-48`) plus `.rname` (`kindel/kindel.py:145`).
 
-`/root/reference` does not exist on the GPU box.  There the only copy is the staged install under
-`baseline/_ref/` (git-ignored; `oracle/stage_reference.py`), used solely by `bench.py`'s CPU legs
-(`--impl reference`, `cpu_baseline`) to time the reference's own functions; the `-m gpu` tests and `smoke()`
-never import this module.  `available()` says whether a reference tree was found.
+Where no reference checkout exists, the only copy is the staged install under `oracle/_ref/`
+(git-ignored; `oracle/stage_reference.py`), used solely by `bench.py`'s CPU legs (`--impl reference`,
+`cpu_baseline`) to time the reference's own functions; the tests and `smoke()` never import this module (they
+compare with the reference's stored results under tests/golden/).  `available()` says whether a reference tree was found.
 
 The decoder here is deliberately independent of the product decoder in `kindel_b200/bamio.py`
 (record-at-a-time `struct.unpack`, no numpy), so the two cross-check each other.
@@ -25,9 +25,9 @@ import types
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # search order: explicit override, the reference tree of the build container, the staged install that
-# travels to the GPU box (baseline/_ref/, produced by oracle/stage_reference.py; git-ignored)
+# stays with the tree (oracle/_ref/, produced by oracle/stage_reference.py; git-ignored)
 _CANDIDATES = [os.environ.get("KINDEL_REFERENCE_ROOT"), "/root/reference",
-               os.path.join(os.path.dirname(_HERE), "baseline", "_ref")]
+               os.path.join(_HERE, "_ref")]
 
 
 def _find_root():

@@ -1,19 +1,14 @@
-"""TEST / BENCH INFRASTRUCTURE ONLY -- stages the UNMODIFIED reference package for the GPU box.
+"""TEST / BENCH INFRASTRUCTURE ONLY -- stages the UNMODIFIED reference package inside the tree.
 
-The reference (bede/kindel v1.2.1) is a pure-Python flit package.  The contract's install
+The reference (bede/kindel v1.2.1) is a pure-Python flit package whose run-time dependencies (simplesam,
+dnaio, argh) need not be installed, so this recipe puts what a `pip install --target` would have put there
+for a pure-Python package -- the package directory `kindel/` with its three modules, byte for byte -- and
+nothing else under `oracle/_ref/`.  `oracle/_ref/` is git-ignored (never part of the repository's history);
+it lets `bench.py --impl reference` / `cpu_baseline` time the reference's own `parse_records` +
+`consensus_sequence` (reference kindel/kindel.py:21-128, 384-430) through `oracle/refload.py`'s import stubs
+on a machine that has no reference checkout.
 
-    python -m pip install --no-index --no-build-isolation --find-links /opt/wheelhouse \
-        --target baseline/_ref /root/reference
-
-fails in this image (build backend `flit_core` is neither installed nor in /opt/wheelhouse; the run-time
-dependencies simplesam / dnaio / argh are absent too), so this recipe produces what that install would have
-put under `baseline/_ref/` for a pure-Python package -- the package directory `kindel/` with its three
-modules, byte for byte -- and nothing else.  `baseline/_ref/` is git-ignored (never part of the repo's
-history) but not gpurun-ignored, so it travels to the GPU box, where `/root/reference` does not exist, and
-`bench.py --impl reference` / `cpu_baseline` can time the reference's own `parse_records` +
-`consensus_sequence` (reference kindel/kindel.py:21-128, 384-430) through `oracle/refload.py`'s import stubs.
-
-    python -m oracle.stage_reference          (also called by __graft_entry__.build() when /root/reference exists)
+    python -m oracle.stage_reference          (also called by __graft_entry__.build(); a no-op without a source)
 """
 from __future__ import annotations
 
@@ -24,12 +19,12 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SRC = os.environ.get("KINDEL_REFERENCE_SRC", "/root/reference")
-DST = os.path.join(ROOT, "baseline", "_ref")
+DST = os.path.join(ROOT, "oracle", "_ref")
 FILES = ("__init__.py", "kindel.py", "cli.py")
 
 
 def stage(verbose: bool = False) -> str | None:
-    """Copy <SRC>/kindel/*.py to baseline/_ref/kindel/.  Returns the staged root, or None if SRC is absent."""
+    """Copy <SRC>/kindel/*.py to oracle/_ref/kindel/.  Returns the staged root, or None if SRC is absent."""
     src_pkg = os.path.join(SRC, "kindel")
     if not os.path.isfile(os.path.join(src_pkg, "kindel.py")):
         return DST if os.path.isfile(os.path.join(DST, "kindel", "kindel.py")) else None
@@ -44,7 +39,7 @@ def stage(verbose: bool = False) -> str | None:
         with open(d, "rb") as fh:
             lines.append("%s  kindel/%s" % (hashlib.sha256(fh.read()).hexdigest(), f))
     with open(os.path.join(DST, "STAGED_FROM.txt"), "w") as fh:
-        fh.write("staged from %s by oracle/stage_reference.py (unmodified; pip --target failed: no flit_core)\n" % SRC)
+        fh.write("staged from %s by oracle/stage_reference.py (unmodified)\n" % SRC)
         fh.write("\n".join(lines) + "\n")
     if verbose:
         print("\n".join(lines), file=sys.stderr)

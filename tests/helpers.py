@@ -1,6 +1,9 @@
 """Shared helpers for the parity tests (test infrastructure)."""
 from __future__ import annotations
 
+import gzip
+import hashlib
+import json
 import os
 import sys
 from collections import OrderedDict
@@ -30,6 +33,47 @@ def reference_alignment_to_table(aln):
     t[8] = aln.clip_ends
     ins = [OrderedDict(d) for d in aln.insertions]
     return t, ins
+
+
+_reference_runs = None
+
+
+def reference_runs():
+    """What the unmodified reference returned on the seeded fuzz inputs and the FASTA files of its suite
+    (tests/golden/reference_runs.json.gz, written by oracle/make_reference_golden.py)."""
+    global _reference_runs
+    if _reference_runs is None:
+        with gzip.open(os.path.join(ROOT, "tests", "golden", "reference_runs.json.gz"), "rt") as fh:
+            _reference_runs = json.load(fh)
+    return _reference_runs
+
+
+def table_sha256(table) -> str:
+    """sha256 of a count table as int32 bytes (the layout of reference_alignment_to_table)."""
+    return hashlib.sha256(np.ascontiguousarray(table, dtype=np.int32).tobytes()).hexdigest()
+
+
+def frame_sha256(df) -> str:
+    """sha256 of a DataFrame's column names, dtypes, index and values: equal digests <=> exactly equal frames."""
+    h = hashlib.sha256()
+    h.update(repr([(str(c), str(t)) for c, t in df.dtypes.items()]).encode())
+    h.update(repr((str(df.index.dtype), df.index.tolist())).encode())
+    for c in df.columns:
+        v = df[c].to_numpy()
+        h.update(repr(v.tolist()).encode() if v.dtype == object else np.ascontiguousarray(v).tobytes())
+    return h.hexdigest()
+
+
+def reference_lists(table, L):
+    """int [19, L+1] table -> the reference's per-position lists (kindel/kindel.py:29-38, 91-96): weights,
+    deletions, clip_start_weights, clip_end_weights, clip_start_depth, clip_end_depth."""
+    t = np.asarray(table).tolist()
+
+    def dicts(row0):
+        return [{b: t[row0 + "ACGTN".index(b)][i] for b in "ATGCN"} for i in range(L)]
+
+    csw, cew = dicts(9), dicts(14)
+    return (dicts(0), t[5], csw, cew, [sum(w[b] for b in "ACGT") for w in csw], [sum(w[b] for b in "ACGT") for w in cew])
 
 
 def event_string(batch, read, q_off, length):

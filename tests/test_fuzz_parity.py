@@ -1,7 +1,7 @@
 """Differential fuzzing of the hot path on random small alignments (tests/fuzz_cases.py).
 
 CPU (always):       C oracle == reference-shaped CPython port, including which exception is raised.
-CPU (container):    C oracle == the UNMODIFIED reference (tables, insertion dicts, FASTA, exceptions).
+CPU (always):       C oracle == what the UNMODIFIED reference returned (tables, insertion dicts, changes, exceptions).
 GPU (`-m gpu`):     engine through the public API == C oracle (tables, events, calls, exceptions)."""
 import numpy as np
 import pytest
@@ -9,7 +9,7 @@ import pytest
 import helpers as H
 from fuzz_cases import random_case
 from kindel_b200 import bamio
-from oracle import coracle, py_oracle, refload, samdecode
+from oracle import coracle, py_oracle, samdecode
 
 N_CASES = 400
 
@@ -82,19 +82,16 @@ def test_c_oracle_vs_python_port(tmp_path):
     assert raised > 20  # the generator really reaches the error paths
 
 
-@pytest.mark.skipif(not refload.available(), reason="reference tree only exists in the build container")
 def test_c_oracle_vs_unmodified_reference(tmp_path):
-    k = refload.load_reference()
+    """The reference's outcome for every case (tests/golden/reference_runs.json.gz, oracle/make_reference_golden.py):
+    the exception it raised, or its tables, insertion dicts in first-seen order and `changes`."""
+    golden = H.reference_runs()["fuzz"]
+    assert len(golden) == N_CASES
     raised = 0
     for seed in range(N_CASES):
         path = _load(tmp_path, seed)
-        try:
-            alns = k.parse_bam(str(path))
-            ref_err = None
-        except IndexError:
-            ref_err = ("IndexError",)
-        except KeyError as exc:
-            ref_err = ("KeyError", exc.args[0])
+        want = golden[seed]
+        ref_err = tuple(want["raises"]) if "raises" in want else None
         try:
             batch = bamio.read_alignment(path)
         except ValueError:
@@ -107,17 +104,16 @@ def test_c_oracle_vs_unmodified_reference(tmp_path):
         if err:
             raised += 1
             continue
-        assert list(alns) == batch.contig_names
+        assert want["contigs"] == batch.contig_names
         ins = H.events_to_dicts(batch, events)
         calls = coracle.vote(counts, 1)
-        for c, aln in enumerate(alns.values()):
-            t, ref_ins = H.reference_alignment_to_table(aln)
-            np.testing.assert_array_equal(H.contig_view(batch, counts, c), t, err_msg=str(seed))
-            s0 = int(batch.contig_slot[c])
-            for i, d in enumerate(ref_ins):
-                assert list(d.items()) == list(ins.get(s0 + i, {}).items()), (seed, i)
-            _, changes = k.consensus_sequence(aln.weights, aln.insertions, aln.deletions, None, False, 1, False)
-            assert H.calls_to_changes(calls[s0:s0 + len(aln.weights)]) == changes, seed
+        for c in range(len(want["contigs"])):
+            t = H.contig_view(batch, counts, c)
+            assert H.table_sha256(t) == want["table_sha256"][c], seed
+            s0, L = int(batch.contig_slot[c]), int(batch.contig_len[c])
+            got_ins = [[i, [list(kv) for kv in ins[s0 + i].items()]] for i in range(L + 1) if ins.get(s0 + i)]
+            assert got_ins == want["insertions"][c], seed
+            assert H.calls_to_changes(calls[s0:s0 + L]) == want["changes"][c], seed
     assert raised > 20
 
 

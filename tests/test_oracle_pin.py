@@ -1,8 +1,7 @@
 """Pins the oracle: the C restatement (oracle/kindel_oracle.c) against
   (a) the golden vectors the UNMODIFIED reference produced (tests/golden/, oracle/make_golden.py), and
-  (b) -- only where /root/reference exists (the build container) -- the reference itself on every
-      fixture of its own test-suite, including the known-answer integers of
-      reference tests/test_kindel.py:63-89.
+  (b) the reference's known-answer integers of its tests/test_kindel.py:63-89 and the FASTA files of its
+      own test-suite (tests/golden/reference_runs.json.gz).
 No GPU involved."""
 import os
 from collections import OrderedDict
@@ -11,9 +10,9 @@ import numpy as np
 import pytest
 
 import helpers as H
-from conftest import golden_input
+from conftest import GOLDEN, golden_input
 from kindel_b200 import bamio
-from oracle import coracle, refload, samdecode
+from oracle import coracle, samdecode
 
 
 def test_golden_tables_insertions_and_vote(manifest, golden_npz):
@@ -94,83 +93,73 @@ def test_oracle_decoder_and_product_decoder_agree(manifest):
             assert H.event_string(batch, k, 0, len(r.seq)) == r.seq.upper() or int(batch.l_seq[k]) >= 0
 
 
-needs_reference = pytest.mark.skipif(not refload.available(), reason="reference tree only exists in the build container")
+def test_reference_known_answers(golden_npz, manifest):
+    """reference tests/test_kindel.py:63-89: the known-answer integers, in the reference's own tables (tests/golden/)
+    and in the C oracle's tables of the same inputs."""
+    def tables(name):
+        batch = bamio.read_alignment(golden_input(manifest["files"][name]))
+        counts, _ = coracle.pileup(batch)
+        assert len(batch.contig_names) == 1
+        return batch, [golden_npz(name)["c0_counts"], H.contig_view(batch, counts, 0)]
+
+    batch, t1 = tables("bwa_1_1")
+    batch2, t2 = tables("ext_3_bc75")
+    assert batch.contig_names == ["ENA|EU155341|EU155341.2"] and int(batch.contig_len[0]) == 9306
+    for t, t_2 in zip(t1, t2):
+        A, G, T, DEL, INS, CLIP_S, CLIP_E = 0, 2, 3, 5, 6, 7, 8
+        assert t.shape[1] == 9307
+        assert t[A, 0] == 22 and t[A, 23] == 57
+        assert t_2[G, 68] == 1 and t_2[T, 2368] == 13
+        assert [t_2[DEL, i] for i in (399, 402, 411, 1048, 1049, 1050)] == [14, 14, 15, 14, 14, 14]
+        assert t_2[CLIP_E, 1748] == 12
+        assert t[CLIP_S, 525] == 16 and t[CLIP_S, 1437] == 84
+        assert t_2[INS, 453] == 14 and t_2[INS, 457] == 14
 
 
-@needs_reference
-def test_reference_known_answers_through_the_oracle_loader():
-    """reference tests/test_kindel.py:63-89, executed against the unmodified module."""
-    k = refload.load_reference()
-    root = os.path.join(refload.REFERENCE_ROOT, "tests")
-    aln = list(k.parse_bam(os.path.join(root, "data_bwa_mem", "1.1.sub_test.bam")).values())[0]
-    aln2 = list(k.parse_bam(os.path.join(root, "data_ext", "3.issue23.bc75.sam")).values())[0]
-    assert aln.ref_id == "ENA|EU155341|EU155341.2" and len(aln.weights) == 9306
-    assert aln.weights[0]["A"] == 22 and aln.weights[23]["A"] == 57
-    assert aln2.weights[68]["G"] == 1 and aln2.weights[2368]["T"] == 13
-    assert [aln2.deletions[i] for i in (399, 402, 411, 1048, 1049, 1050)] == [14, 14, 15, 14, 14, 14]
-    assert aln2.clip_ends[1748] == 12
-    assert aln.clip_starts[525] == 16 and aln.clip_starts[1437] == 84
-    assert sum(aln2.insertions[453].values()) == 14 and sum(aln2.insertions[457].values()) == 14
-
-
-@needs_reference
 def test_c_oracle_equals_reference_on_every_reference_fixture():
-    """All 17 BAM/SAM fixtures of the reference's test-suite (bact.tiny excluded: 50 s in the
-    reference): tables, insertion dicts with their first-seen order, and the vote."""
-    import glob
-
-    k = refload.load_reference()
-    root = os.path.join(refload.REFERENCE_ROOT, "tests")
-    files = sorted(glob.glob(root + "/data_*/*.bam") + glob.glob(root + "/data_*/*.sam"))
-    files = [f for f in files if "bact" not in f]
-    assert len(files) == 17
-    for path in files:
-        batch = bamio.read_alignment(path)
+    """The first records of all 17 BAM/SAM fixtures of the reference's test-suite, byte for byte as the aligners
+    wrote them (read names, qualities, aux tags; tests/golden/inputs/cut_*), through the product decoder and the C
+    oracle == what the reference returned for them (oracle/make_reference_golden.py): tables, insertion dicts with
+    their first-seen order, and the vote."""
+    cuts = H.reference_runs()["cuts"]
+    assert len(cuts) == 17
+    for name, want in cuts.items():
+        assert "raises" not in want, name
+        batch = bamio.read_alignment(os.path.join(GOLDEN, want["input"]))
         counts, events = coracle.pileup(batch)
         calls = coracle.vote(counts, 1)
         ins = H.events_to_dicts(batch, events)
-        alns = k.parse_bam(path)
-        assert list(alns) == batch.contig_names
-        for c, aln in enumerate(alns.values()):
-            t, ref_ins = H.reference_alignment_to_table(aln)
-            np.testing.assert_array_equal(H.contig_view(batch, counts, c), t, err_msg=path)
-            s0 = int(batch.contig_slot[c])
-            for i, d in enumerate(ref_ins):
-                assert list(d.items()) == list(ins.get(s0 + i, {}).items())
-            _, changes = k.consensus_sequence(aln.weights, aln.insertions, aln.deletions, None, False, 1, False)
-            assert H.calls_to_changes(calls[s0:s0 + len(aln.weights)]) == changes
+        assert batch.contig_names == want["contigs"], name
+        for c in range(len(want["contigs"])):
+            assert H.table_sha256(H.contig_view(batch, counts, c)) == want["table_sha256"][c], name
+            s0, L = int(batch.contig_slot[c]), int(batch.contig_len[c])
+            got_ins = [[i, [list(kv) for kv in ins[s0 + i].items()]] for i in range(L + 1) if ins.get(s0 + i)]
+            assert got_ins == want["insertions"][c], name
+            assert H.calls_to_changes(calls[s0:s0 + L]) == want["changes"][c], name
 
 
-@needs_reference
-def test_golden_fasta_files_of_the_reference_suite():
-    """The reference's own golden FASTA files (plain + realign), via the oracle loader: 21 of 22,
-    the 22nd belongs to a test the reference has commented out (tests/test_kindel.py:281-299)."""
-    import glob
+def test_golden_fasta_files_of_the_reference_suite(manifest):
+    """The reference's own golden FASTA files (plain + realign; tests/golden/reference_runs.json.gz) against oracle
+    tables + host code: 21 of 22, the 22nd belongs to a test the reference has commented out
+    (tests/test_kindel.py:281-299) and the reference itself does not reproduce it."""
+    from kindel_b200 import kindel as K
 
-    k = refload.load_reference()
-    root = os.path.join(refload.REFERENCE_ROOT, "tests")
-
-    def fasta(path):
-        recs, name = {}, None
-        for line in open(path):
-            line = line.strip()
-            if line.startswith(">"):
-                name = line[1:]
-                recs[name] = ""
-            elif name:
-                recs[name] += line
-        return recs
-
+    fasta = H.reference_runs()["fasta"]
+    assert len(fasta) == 11
     ok, bad = 0, []
-    for d, ext in (("data_bwa_mem", ".bam"), ("data_minimap2", ".bam"), ("data_ext", ".sam")):
-        for p in sorted(glob.glob(os.path.join(root, d, "*" + ext))):
-            for realign, suf in ((False, ".fa"), (True, ".realign.fa")):
-                res = k.bam_to_consensus(p, realign, 1, 7, 0.1, 50, False, False)
-                if {r.name: r.sequence for r in res.consensuses} == fasta(os.path.splitext(p)[0] + suf):
-                    ok += 1
-                else:
-                    bad.append(os.path.basename(p) + suf)
-    assert ok == 21 and bad == ["3.issue23.bc75.sam.realign.fa"]
+    for name, want in sorted(fasta.items()):
+        path = golden_input(manifest["files"][name])
+        batch = bamio.read_alignment(path)
+        counts, events = coracle.pileup(batch)
+        run = K.PileupRun.from_host_tables(batch, counts, coracle.derive(counts), events)
+        for realign in (False, True):
+            kind = "realign" if realign else "plain"
+            res = K.consensus_from_run(run, coracle.vote(counts, 1), path, realign, 1, 7, 0.1, 50, False, False)
+            if {r.name: r.sequence for r in res.consensuses} == want[kind]:
+                ok += 1
+            else:
+                bad.append((name, kind))
+    assert ok == 21 and bad == [("ext_3_bc75", "realign")]
 
 
 def test_python_port_against_golden(manifest, golden_npz):
