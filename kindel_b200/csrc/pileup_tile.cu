@@ -30,10 +30,9 @@ namespace kdl {
 
 constexpr int W_CONSUMERS = 8;   // consumer warps (one 64-slot window each)
 constexpr int W_PRODUCERS = 4;   // producer warps
-#ifndef KDL_W_STAGES
-#define KDL_W_STAGES 2  // measured on B200 (cfg 4): 2 stages 0.216 ms, 3 stages 0.243 ms, 4 stages 0.262 ms -- see TileCfg
-#endif
-constexpr int W_STAGES = KDL_W_STAGES;  // depth of the shared-memory ring
+// depth of the shared-memory ring.  Measured on B200 (cfg 4, all simple): 2 stages 0.216 ms, 3 stages 0.243 ms,
+// 4 stages 0.262 ms for K0 + K1 -- see TileCfg and profiles/r02_ring_depth.txt
+constexpr int W_STAGES = 2;
 constexpr int W_THREADS = 32 * (W_CONSUMERS + W_PRODUCERS);
 constexpr int W_PT = 32 * W_PRODUCERS;  // producer threads
 // setmaxnreg per role: 128 * kProducer + 256 * kConsumer <= 384 * 80 (the launch bound's allocation)
@@ -46,9 +45,8 @@ static_assert(W_PT * TileRegs<true>::kProducer + 32 * W_CONSUMERS * TileRegs<tru
 template <bool kCx> struct TileCfg;
 // An item is sized so that the whole ring fits half an SM's shared memory.  A tile of deep short-read data is
 // several items, each a sub-range of the tile's (sorted) reads, and every item costs each consumer warp a wait, a
-// search and a partly filled last block: FEW LARGE items beat a deeper ring of small ones (the 3- and 4-stage
-// configurations are kept for that measurement, profiles/r02_ring_depth.txt).
-#if KDL_W_STAGES == 2
+// search and a partly filled last block: FEW LARGE items beat a deeper ring of small ones (3 and 4 stages with
+// proportionally smaller items were measured slower, profiles/r02_ring_depth.txt).
 template <> struct TileCfg<false> {
     static constexpr int kRmax = 512;    // reads per item
     static constexpr int kCapW = 9728;   // words of seq4 per item (38 KB: ~510 reads of 150 bases)
@@ -59,31 +57,6 @@ template <> struct TileCfg<true> {
     static constexpr int kCapW = 7680;   // 30 KB
     static constexpr int kPcap = 672;
 };
-#elif KDL_W_STAGES == 3
-template <> struct TileCfg<false> {
-    static constexpr int kRmax = 384;
-    static constexpr int kCapW = 6144;   // 24 KB
-    static constexpr int kPcap = 0;
-};
-template <> struct TileCfg<true> {
-    static constexpr int kRmax = 256;
-    static constexpr int kCapW = 5120;   // 20 KB
-    static constexpr int kPcap = 448;
-};
-#elif KDL_W_STAGES == 4
-template <> struct TileCfg<false> {
-    static constexpr int kRmax = 256;
-    static constexpr int kCapW = 4736;   // 18.5 KB: ~250 reads of 150 bases
-    static constexpr int kPcap = 0;
-};
-template <> struct TileCfg<true> {
-    static constexpr int kRmax = 256;
-    static constexpr int kCapW = 3328;   // 13 KB
-    static constexpr int kPcap = 320;
-};
-#else
-#error "KDL_W_STAGES must be 2, 3 or 4"
-#endif
 
 enum : int { ITEM_FIRST = 1, ITEM_LAST = 2, ITEM_EMPTY = 4, ITEM_END = 8 };
 
@@ -177,7 +150,7 @@ pileup_tile_kernel(kdl_batch b, int32_t* __restrict__ counts, long long n_slots,
         uint32_t pph = 0;     // parity of that slot's round (flips when ps wraps)
         bool wrapped = false;
         auto acquire_stage = [&]() -> Stage& {
-            if (wrapped) mbar_wait_relaxed(&sm.empty[ps], pph ^ 1u);  // consumers released its last use
+            if (wrapped) mbar_wait(&sm.empty[ps], pph ^ 1u);  // consumers released its last use
             return sm.st[ps];
         };
         auto publish = [&]() {  // this warp's part of the item is written; on to the next ring slot

@@ -132,26 +132,11 @@ __device__ __forceinline__ void cp_async4(void* dst, const void* src) {
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
-#ifndef KDL_WAIT_HINT_NS
-#define KDL_WAIT_HINT_NS 0     // > 0: try_wait may suspend the thread for up to this long before it reports failure
-#endif
-#ifndef KDL_WAIT_SLEEP_NS
-#define KDL_WAIT_SLEEP_NS 0    // > 0: producers sleep this long between two failed polls (consumers always poll)
-#endif
-template <int kHintNs>
-__device__ __forceinline__ bool mbar_try(uint64_t* bar, uint32_t parity) {
+// Plain polling: a nanosleep between polls or a suspend-time hint on try_wait measured the same to four digits, for
+// producers and consumers alike (profiles/r02_ring_depth.txt).
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     uint32_t done;
-    if (kHintNs > 0) {
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n"
-            "selp.u32 %0, 1, 0, p;\n"
-            "}\n"
-            : "=r"(done)
-            : "r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)kHintNs)
-            : "memory");
-    } else {
+    do {
         asm volatile(
             "{\n"
             ".reg .pred p;\n"
@@ -161,23 +146,7 @@ __device__ __forceinline__ bool mbar_try(uint64_t* bar, uint32_t parity) {
             : "=r"(done)
             : "r"(smem_u32(bar)), "r"(parity)
             : "memory");
-    }
-    return done != 0;
-}
-#ifndef KDL_WAIT_SLEEP_CONS_NS
-#define KDL_WAIT_SLEEP_CONS_NS 0   // > 0: the same for the consumers' waits
-#endif
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    while (!mbar_try<KDL_WAIT_HINT_NS>(bar, parity)) {
-        if (KDL_WAIT_SLEEP_CONS_NS > 0) __nanosleep(KDL_WAIT_SLEEP_CONS_NS);
-    }
-}
-// the same for a waiter that is in nobody's way (a producer waiting for a free stage): its polls must not take issue
-// slots from the warps that count
-__device__ __forceinline__ void mbar_wait_relaxed(uint64_t* bar, uint32_t parity) {
-    while (!mbar_try<KDL_WAIT_HINT_NS>(bar, parity)) {
-        if (KDL_WAIT_SLEEP_NS > 0) __nanosleep(KDL_WAIT_SLEEP_NS);
-    }
+    } while (!done);
 }
 #endif  // KDL_HOST_EMU
 
@@ -203,22 +172,10 @@ template <int kRegs> __device__ __forceinline__ void reg_dealloc() { asm volatil
 template <int kRegs> __device__ __forceinline__ void reg_alloc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kRegs)); }
 #endif  // KDL_HOST_EMU
 
-// first index i in [0, n) with g[i] >= key (n if none); g sorted, n <= 1024, whole warp calls
-__device__ __forceinline__ int lower_bound_warp(const int* g, int n, int key, int lane) {
-    const int step = (n + 31) >> 5;  // <= 32
-    if (step == 0) return 0;
-    const int i1 = (lane + 1) * step - 1;
-    const unsigned m1 = __ballot_sync(0xffffffffu, i1 < n ? g[i1] >= key : true);
-    if (m1 == 0u) return n;       // every probed element (incl. the last one) is < key
-    const int k = __ffs(m1) - 1;  // first bucket whose last element is >= key
-    const int i2 = k * step + lane;
-    const unsigned m2 = __ballot_sync(0xffffffffu, (lane < step && i2 < n) ? g[i2] >= key : true);
-    const int r = k * step + __ffs(m2) - 1;
-    return r < n ? r : n;
-}
-
-// the same for TWO keys at once (key_a <= key_e): one probe load serves both searches and the two dependent
-// chains (load -> ballot -> load -> ballot) overlap
+// first index i in [0, n) with g[i] >= key (n if none), for TWO keys at once (key_a <= key_e); g sorted,
+// n <= 1024, whole warp calls.  Two 32-ary rounds: the lanes probe the last element of 32 buckets, then the
+// elements of the first bucket whose last element is >= key.  One probe load serves both searches and the two
+// dependent chains (load -> ballot -> load -> ballot) overlap.
 __device__ __forceinline__ void lower_bound_warp2(const int* g, int n, int key_a, int key_e, int lane, int& ra, int& re) {
     const int step = (n + 31) >> 5;  // <= 32
     if (step == 0) { ra = re = 0; return; }
@@ -250,25 +207,9 @@ struct Planes {
 #pragma unroll
         for (int k = 0; k < F_P; ++k) p[k] = 0;
     }
-    // Harley-Seal: 8 one-bit-per-counter inputs -> 7 full adders + a ripple from the 8s plane up
-    __device__ __forceinline__ void add8(const uint32_t (&x)[8]) {
-        uint32_t ta, tb, tc, td, fa, fb, e;
-        csa(ta, p[0], p[0], x[0], x[1]);
-        csa(tb, p[0], p[0], x[2], x[3]);
-        csa(fa, p[1], p[1], ta, tb);
-        csa(tc, p[0], p[0], x[4], x[5]);
-        csa(td, p[0], p[0], x[6], x[7]);
-        csa(fb, p[1], p[1], tc, td);
-        csa(e, p[2], p[2], fa, fb);
-#pragma unroll
-        for (int k = 3; k < F_P; ++k) {
-            const uint32_t t = p[k] & e;
-            p[k] ^= e;
-            e = t;
-        }
-    }
-    // kLean: the same 7 full adders, but the carry out of the 4s plane (weight 8) is handed back instead of being
-    // rippled up; the caller pairs two of them with one more full adder, so the ripple runs once per 16 reads
+    // Harley-Seal: 8 one-bit-per-counter inputs -> 7 full adders.  The carry out of the 4s plane (weight 8) is
+    // handed back instead of being rippled up; the caller pairs two of them with one more full adder, so the
+    // ripple runs once per 16 reads
     __device__ __forceinline__ uint32_t add8_carry(const uint32_t (&x)[8]) {
         uint32_t ta, tb, tc, td, fa, fb, e;
         csa(ta, p[0], p[0], x[0], x[1]);

@@ -389,7 +389,6 @@ inline void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) 
 inline void mbar_wait(uint64_t* bar, uint32_t parity) {
     while (reinterpret_cast<MbarBits*>(bar)->phase == (parity & 1u)) emu::yield();
 }
-inline void mbar_wait_relaxed(uint64_t* bar, uint32_t parity) { mbar_wait(bar, parity); }
 inline void mbar_arrive(uint64_t* bar) {  // mbarrier.arrive: one arrival, no bytes
     MbarBits* b = reinterpret_cast<MbarBits*>(bar);
     if (b->pending == 0) emu::fail("emulator: mbarrier arrival beyond its count");

@@ -16,9 +16,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 EMU_DIR = os.path.join(ROOT, "tests", "emu")
 OUT_DIR = os.path.join(EMU_DIR, "_build")
-# KDL_EMU_DEFS="-DKDL_W_STAGES=2" builds (and loads) a variant of the emulated kernels next to the default one
-EXTRA_DEFS = os.environ.get("KDL_EMU_DEFS", "").split()
-LIB = os.path.join(OUT_DIR, "libkdl_emu%s.so" % "".join(c if c.isalnum() else "_" for c in "".join(EXTRA_DEFS)))
+LIB = os.path.join(OUT_DIR, "libkdl_emu.so")
 CUDA_INCLUDE = os.environ.get("CUDA_INCLUDE", "/usr/local/cuda/include")
 F_STORE, F_ADD, F_ATOMIC = 0, 1, 2  # flush modes of the tile kernel (tile_common.cuh)
 
@@ -45,7 +43,7 @@ def load():
     if not (os.path.exists(LIB) and all(os.path.getmtime(s) <= os.path.getmtime(LIB) for s in src)):
         os.makedirs(OUT_DIR, exist_ok=True)
         cmd = ["g++", "-std=c++17", "-O1", "-g", "-fPIC", "-shared", "-I", CUDA_INCLUDE, "-I", os.path.join(ROOT, "include"),
-               *EXTRA_DEFS, os.path.join(EMU_DIR, "emu_pileup.cpp"), "-o", LIB]
+               os.path.join(EMU_DIR, "emu_pileup.cpp"), "-o", LIB]
         res = subprocess.run(cmd, capture_output=True, text=True)
         if res.returncode != 0:
             raise RuntimeError("building the kernel emulator failed:\n" + res.stdout + res.stderr)

@@ -257,19 +257,3 @@ def test_other_thread_interleavings(schedule, seed):
         np.testing.assert_array_equal(got_e, want_e)
     finally:
         E.set_schedule("forward")
-
-
-@pytest.mark.parametrize("stages", [3, 4])
-def test_deeper_rings_stay_correct(stages):
-    """The 3- and 4-stage configurations of the tile kernel (kept for the ring-depth measurement,
-    profiles/r02_ring_depth.txt) are built with -DKDL_W_STAGES and must reproduce the oracle on the same cases."""
-    import os
-    import subprocess
-    import sys
-
-    env = dict(os.environ, KDL_EMU_DEFS="-DKDL_W_STAGES=%d" % stages)
-    res = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-q", "-x", "-p", "no:cacheprovider",
-                          "-k", "(tile_owner and (deep or cfg4_like or sparse)) or (complex_reads_in_the_tile and 3)"],
-                         env=env, capture_output=True, text=True, timeout=1500, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    assert res.returncode == 0, res.stdout[-2000:] + res.stderr[-2000:]
-    assert " passed" in res.stdout
