@@ -23,7 +23,6 @@ with a 2-process gloo group on CPU in tests/test_distributed_cpu.py.
 from __future__ import annotations
 
 import ctypes as C
-import math
 import os
 
 import numpy as np
@@ -325,7 +324,7 @@ class ShardedConsensus:
         if self.mode == "fused":
             st = int(torch.cuda.current_stream(self.device).cuda_stream)
             with torch.cuda.device(self.device):
-                _ffi.check(self.lib.kdl_exchange_vote(C.byref(self.xstruct[par]), self.n_slots, int(math.ceil(min_depth)),
+                _ffi.check(self.lib.kdl_exchange_vote(C.byref(self.xstruct[par]), self.n_slots, engine.min_depth_ceil(min_depth),
                                                       self.epoch, st), "kdl_exchange_vote")
                 _ffi.check(self.lib.kdl_exchange_wait(C.byref(self.xstruct[par]), self.epoch, st), "kdl_exchange_wait")
             return self.tables.calls[par]
@@ -341,7 +340,7 @@ class ShardedConsensus:
         with torch.cuda.device(self.device):
             rc = self.lib.kdl_vote_peers_sparse(
                 self.ptr_arr[par], self.foot_lo, self.foot_hi, self.world, self.n_slots, lo, hi,
-                int(math.ceil(min_depth)), calls.data_ptr(), None,
+                engine.min_depth_ceil(min_depth), calls.data_ptr(), None,
                 int(torch.cuda.current_stream(self.device).cuda_stream))
         _ffi.check(rc, "kdl_vote_peers_sparse")
         # 1 byte per slot; also the fence after which peers may overwrite this parity's tables again

@@ -189,6 +189,23 @@ def diagnose_and_raise(dbatch: DeviceBatch):
     raise RuntimeError("pileup raised its error flag but no offending read was found")
 
 
+MIN_DEPTH_CLAMP = 2 ** 62
+
+
+def min_depth_ceil(min_depth) -> int:
+    """The int64 the vote kernels compare an integer depth with: `depth < min_depth` (kindel.py:415) is
+    `depth < ceil(min_depth)`.  nan compares false with everything, so it never calls N; +-inf and finite values
+    beyond int64 are clamped to +-2**62.  Depth sums are at most 5 * (2**31 - 1), so the clamp changes no answer."""
+    md = float(min_depth)
+    if math.isnan(md):
+        return -MIN_DEPTH_CLAMP
+    if md >= MIN_DEPTH_CLAMP:
+        return MIN_DEPTH_CLAMP
+    if md <= -MIN_DEPTH_CLAMP:
+        return -MIN_DEPTH_CLAMP
+    return int(math.ceil(md))
+
+
 def vote(counts: torch.Tensor, min_depth=1, out: torch.Tensor = None) -> torch.Tensor:
     """K2.  counts int32[>=7, n_slots] (contiguous) -> calls uint8[n_slots] (`out` reuses a buffer)."""
     lib = _ffi.load()
@@ -196,7 +213,7 @@ def vote(counts: torch.Tensor, min_depth=1, out: torch.Tensor = None) -> torch.T
     n_slots = counts.shape[1]
     with torch.cuda.device(dev):
         calls = out if out is not None else torch.empty(n_slots, dtype=torch.uint8, device=dev)
-        rc = lib.kdl_vote(counts.data_ptr(), n_slots, int(math.ceil(min_depth)), calls.data_ptr(),
+        rc = lib.kdl_vote(counts.data_ptr(), n_slots, min_depth_ceil(min_depth), calls.data_ptr(),
                           _stream_ptr(dev))
         _ffi.check(rc, "kdl_vote")
     return calls
@@ -297,7 +314,7 @@ class HostContext:
             calls_out = np.empty(host.n_slots, dtype=np.uint8)
         diag = _ffi.KdlDiag()
         rc = self._lib.kdl_ctx_consensus(
-            self._h, C.byref(struct), host.n_slots, host.n_events, int(math.ceil(min_depth)),
+            self._h, C.byref(struct), host.n_slots, host.n_events, min_depth_ceil(min_depth),
             calls_out.ctypes.data, counts_out.ctypes.data if counts_out is not None else None,
             events_out.ctypes.data if (events_out is not None and host.n_events) else None, C.byref(diag))
         if rc in (_ffi.KDL_ERR_INDEX, _ffi.KDL_ERR_KEY):

@@ -116,12 +116,22 @@ def pileup(batch, counts=None):
     return counts, events[: n_evt.value]
 
 
+def _min_depth_ceil(min_depth):
+    """`depth < min_depth` (reference kindel.py:415) as `depth < ceil(min_depth)` over int64.  Written out here
+    rather than taken from the engine, so the oracle stays an independent side of the comparison: nan never
+    calls N; +-inf and values beyond int64 clamp to +-2**62, far outside any depth sum."""
+    md = float(min_depth)
+    if md != md:
+        return -(2 ** 62)
+    return int(math.ceil(min(max(md, -2.0 ** 62), 2.0 ** 62)))
+
+
 def vote(counts, min_depth=1):
     lib = _load()
     counts = np.ascontiguousarray(counts, dtype=np.int32)
     n_slots = counts.shape[1]
     calls = np.zeros(n_slots, dtype=np.uint8)
-    lib.oracle_vote(counts.ctypes.data, n_slots, int(math.ceil(min_depth)), calls.ctypes.data)
+    lib.oracle_vote(counts.ctypes.data, n_slots, _min_depth_ceil(min_depth), calls.ctypes.data)
     return calls
 
 

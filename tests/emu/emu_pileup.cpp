@@ -11,6 +11,7 @@
 #include "../../kindel_b200/csrc/pileup_general.cu"
 #include "../../kindel_b200/csrc/pileup_simple.cu"
 #include "../../kindel_b200/csrc/vote.cu"
+#include "../../kindel_b200/csrc/assemble.cu"
 
 static char g_error[512];
 
@@ -103,6 +104,30 @@ int emu_vote(const int32_t* counts, long long n_slots, long long min_depth_ceil,
 int emu_derive(const int32_t* counts, long long n_slots, int32_t* out) {
     g_error[0] = 0;
     EMU_RUN((n_slots + 255) / 256, 256, kdl::derive_kernel(counts, n_slots, out));
+    return 0;
+}
+// K4 over slots [slot_lo, slot_hi), one thread per slot as kdl_cdr_flags launches it
+int emu_cdr_flags(const int32_t* counts, long long n_slots, long long slot_lo, long long slot_hi, double decay,
+                  uint8_t* flags, uint8_t* bases) {
+    g_error[0] = 0;
+    if (slot_hi <= slot_lo) return 0;
+    EMU_RUN((slot_hi - slot_lo + 255) / 256, 256,
+            kdl::cdr_flags_kernel(counts, n_slots, slot_lo, slot_hi, decay, flags, bases));
+    return 0;
+}
+// K5: block sums, the one-CTA scan over them, the scatter -- the grids of kdl_assemble.  block_sums holds
+// kdl_assemble_scratch_words(n_slots) words, offsets n_slots + 1.
+int emu_assemble(const uint8_t* calls, long long n_slots, const int64_t* contig_slot, const int32_t* contig_len,
+                 int n_contigs, const int64_t* ins_slot, const uint32_t* ins_off, const uint8_t* ins_bytes, long long n_ins,
+                 uint32_t* block_sums, uint32_t* offsets, uint8_t* out) {
+    g_error[0] = 0;
+    kdl::AssembleArgs a;
+    a.calls = calls; a.n_slots = n_slots; a.contig_slot = contig_slot; a.contig_len = contig_len; a.n_contigs = n_contigs;
+    a.ins_slot = ins_slot; a.ins_off = ins_off; a.ins_bytes = ins_bytes; a.n_ins = n_ins;
+    const long long n_blocks = (n_slots + 1 + kdl::A_BLOCK - 1) / kdl::A_BLOCK;
+    EMU_RUN(n_blocks, kdl::A_THREADS, kdl::assemble_sums_kernel(a, block_sums));
+    EMU_RUN(1, kdl::A_THREADS, kdl::assemble_scan_sums_kernel(block_sums, n_blocks));
+    EMU_RUN(n_blocks, kdl::A_THREADS, kdl::assemble_scatter_kernel(a, block_sums, offsets, out));
     return 0;
 }
 // K2p: vote over the SUM of several tables, each non-zero only inside its footprint [lo, hi)

@@ -32,7 +32,7 @@ def _sources():
     return [os.path.join(EMU_DIR, "cuda_emu.h"), os.path.join(EMU_DIR, "emu_pileup.cpp"),
             os.path.join(csrc, "kdl_common.cuh"), os.path.join(csrc, "tile_common.cuh"), os.path.join(csrc, "pileup_tile.cu"),
             os.path.join(csrc, "pileup_general.cu"), os.path.join(csrc, "pileup_simple.cu"), os.path.join(csrc, "vote.cu"),
-            os.path.join(ROOT, "include", "kindel_b200.h")]
+            os.path.join(csrc, "assemble.cu"), os.path.join(ROOT, "include", "kindel_b200.h")]
 
 
 def load():
@@ -62,6 +62,8 @@ def load():
     lib.emu_derive.argtypes = [vp, C.c_longlong, vp]
     lib.emu_vote_peers.argtypes = [C.POINTER(vp), C.POINTER(C.c_longlong), C.POINTER(C.c_longlong), C.c_int,
                                    C.c_longlong, C.c_longlong, C.c_longlong, C.c_longlong, vp, vp]
+    lib.emu_cdr_flags.argtypes = [vp, C.c_longlong, C.c_longlong, C.c_longlong, C.c_double, vp, vp]
+    lib.emu_assemble.argtypes = [vp, C.c_longlong, vp, vp, C.c_int, vp, vp, vp, C.c_longlong, vp, vp, vp]
     lib.emu_set_schedule.argtypes = [C.c_int, C.c_ulonglong]
     lib.emu_set_schedule.restype = None
     lib.emu_exchange_epoch.argtypes = [C.POINTER(_ffi.KdlExchange), C.c_int, C.c_longlong, C.c_longlong, C.c_int, C.c_int]
@@ -160,12 +162,12 @@ def pileup_pipeline(batch, grid: int = 3, split: int = 1):
 
 
 def vote(counts: np.ndarray, min_depth=1) -> np.ndarray:
-    import math
+    from kindel_b200 import engine
 
     lib = load()
     counts = np.ascontiguousarray(counts, dtype=np.int32)
     calls = np.zeros(counts.shape[1], dtype=np.uint8)
-    _check(lib.emu_vote(counts.ctypes.data, counts.shape[1], int(math.ceil(min_depth)), calls.ctypes.data))
+    _check(lib.emu_vote(counts.ctypes.data, counts.shape[1], engine.min_depth_ceil(min_depth), calls.ctypes.data))
     return calls
 
 
@@ -177,9 +179,49 @@ def derive(counts: np.ndarray) -> np.ndarray:
     return out
 
 
+def cdr_flags(counts: np.ndarray, slot_lo: int, slot_hi: int, clip_decay_threshold: float):
+    """K4 over slots [slot_lo, slot_hi): (flags uint8, bases uint8) of those slots, like engine.cdr_flags."""
+    lib = load()
+    counts = np.ascontiguousarray(counts, dtype=np.int32)
+    n_slots = counts.shape[1]
+    flags = np.full(n_slots, 0xEE, dtype=np.uint8)  # (a slot the kernel skips keeps the marker)
+    bases = np.full(n_slots, 0xEE, dtype=np.uint8)
+    _check(lib.emu_cdr_flags(counts.ctypes.data, n_slots, int(slot_lo), int(slot_hi), float(clip_decay_threshold),
+                             flags.ctypes.data, bases.ctypes.data))
+    return flags[slot_lo:slot_hi].copy(), bases[slot_lo:slot_hi].copy()
+
+
+def assemble(calls: np.ndarray, contig_slot, contig_len, ins_slots, ins_strings, want_offsets=False):
+    """K5 over host buffers, like engine.assemble: the consensus text of every contig (list of str); with
+    want_offsets also the offsets array [n_slots + 1] the scatter wrote."""
+    lib = load()
+    calls = np.ascontiguousarray(calls, dtype=np.uint8)
+    n_slots = calls.shape[0]
+    slot = np.ascontiguousarray(contig_slot, dtype=np.int64)
+    length = np.ascontiguousarray(contig_len, dtype=np.int32)
+    enc = [x.encode("ascii") for x in ins_strings]
+    ins_off = np.zeros(len(enc) + 1, dtype=np.uint32)
+    if enc:
+        ins_off[1:] = np.cumsum([len(x) for x in enc])
+    blob = np.frombuffer(b"".join(enc) or b"\0", dtype=np.uint8).copy()
+    ins_slot = np.ascontiguousarray(ins_slots, dtype=np.int64) if enc else np.zeros(1, dtype=np.int64)
+    n_blocks = (n_slots + 1 + 1023) // 1024
+    sums = np.full(n_blocks + 1, 0xDEADBEEF, dtype=np.uint32)
+    offsets = np.full(n_slots + 1, 0xDEADBEEF, dtype=np.uint32)
+    out = np.zeros(n_slots + int(ins_off[-1]) + 16, dtype=np.uint8)
+    _check(lib.emu_assemble(calls.ctypes.data, n_slots, slot.ctypes.data, length.ctypes.data, len(slot),
+                            ins_slot.ctypes.data, ins_off.ctypes.data, blob.ctypes.data, len(enc), sums.ctypes.data,
+                            offsets.ctypes.data, out.ctypes.data))
+    starts = offsets[slot].astype(np.int64)
+    ends = offsets[slot + length.astype(np.int64)].astype(np.int64)
+    text = out[: int(offsets[n_slots])].tobytes()
+    texts = [text[a:b].decode("ascii") for a, b in zip(starts.tolist(), ends.tolist())]
+    return (texts, offsets) if want_offsets else texts
+
+
 def vote_peers(tables, feet, slot_lo, slot_hi, min_depth=1, want_reduced=False):
     """K2p over host tables: vote of the SUM of `tables` on [slot_lo, slot_hi); feet = [(lo, hi)] or None."""
-    import math
+    from kindel_b200 import engine
 
     lib = load()
     n = len(tables)
@@ -189,7 +231,7 @@ def vote_peers(tables, feet, slot_lo, slot_hi, min_depth=1, want_reduced=False):
     hi = (C.c_longlong * n)(*[f[1] for f in feet]) if feet else None
     calls = np.zeros(n_slots, dtype=np.uint8)
     reduced = np.zeros((7, n_slots), dtype=np.int32) if want_reduced else None
-    _check(lib.emu_vote_peers(ptrs, lo, hi, n, n_slots, slot_lo, slot_hi, int(math.ceil(min_depth)), calls.ctypes.data,
+    _check(lib.emu_vote_peers(ptrs, lo, hi, n, n_slots, slot_lo, slot_hi, engine.min_depth_ceil(min_depth), calls.ctypes.data,
                               reduced.ctypes.data if want_reduced else None))
     return (calls, reduced) if want_reduced else calls
 
@@ -198,9 +240,7 @@ def exchange_epoch(tables, feet, slices, calls, flags, epoch, min_depth=1, grid=
     """One epoch of the fused multi-GPU exchange (K2x on every rank, then K2g on every rank) with the ranks'
     buffers in host memory.  tables[r]: int32 [19, n_slots]; calls[r]: uint8 [n_slots]; flags: dict of per-rank
     int32 arrays 'ready', 'done' (16 each) and 'counter' (1), persistent across epochs."""
-    import math
-
-    from kindel_b200 import _ffi
+    from kindel_b200 import _ffi, engine
 
     lib = load()
     n = len(tables)
@@ -217,7 +257,7 @@ def exchange_epoch(tables, feet, slices, calls, flags, epoch, min_depth=1, grid=
             x.foot_lo[p], x.foot_hi[p] = feet[p]
             x.slice_lo[p], x.slice_hi[p] = slices[p]
         x.counter = flags["counter"][r].ctypes.data
-    _check(lib.emu_exchange_epoch(xs, n, n_slots, int(math.ceil(min_depth)), epoch, grid))
+    _check(lib.emu_exchange_epoch(xs, n, n_slots, engine.min_depth_ceil(min_depth), epoch, grid))
 
 
 def set_schedule(mode: str = "forward", seed: int = 1):
